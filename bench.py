@@ -7,11 +7,19 @@ Default workload (N=1): BASELINE configs[1] -- "VmambaIR-light SRx4 inference, B
 (full SR net training step, 4 img/GPU, gradient all-reduce over NCCL).  Images shard on the batch axis: every
 rank processes its own batch (weak scaling), inference has no collective.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload infer|train]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload infer|train] [--dump-outputs DIR]
   torchrun --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 One JSON line on rank 0.  `--impl reference` times the CPU oracle port of the reference path (oracle/),
 rank 0 only, one image per step.
+
+--dump-outputs DIR: rank 0 writes what the timed path computed in its last timed step as DIR/<name>.npy (float32), so that
+two builds run with the same arguments (same seeded inputs and weights) can be compared output for output:
+  sr            the SR output batch (N x 3 x 4H x 4W) of the inference engine (--impl reference: of image 0 through the oracle)
+  train_loss    the L1 loss of the training step (--workload train, and the training sub-record of the default run)
+  train_params  the flat fp32 parameter buffer after that step's optimizer update
+Two runs of one build already differ slightly (fp32 atomics in the out_norm statistics and the backward, then bf16 storage
+over 27 blocks: max |diff| of sr 0.032 between two runs on one B200 at its 1000 W limit), so compare with a tolerance.
 """
 import argparse
 import json
@@ -25,11 +33,24 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 B_PER_GPU_INFER = 8
 B_PER_GPU_TRAIN = 4
 H = W = 64
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(outputs, out_dir):
+    """outputs: name -> tensor; written as out_dir/<name>.npy in float32"""
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in outputs.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: outputs to dump ({total} bytes) exceed {DUMP_LIMIT_BYTES} bytes")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
 
 
 def env_rank():
@@ -149,12 +170,14 @@ def cpu_oracle_images_per_s(steps, warmup, threads=None, x=None, kind="light"):
     return 1.0 / mean, mean, y
 
 
-def run_reference(args):
+def run_reference(args, outputs=None):
     rank, _, world = env_rank()
     if rank != 0:
         return
     cores = os.cpu_count()
-    ips, mean, _ = cpu_oracle_images_per_s(args.steps, args.warmup, kind=args.net)
+    ips, mean, y = cpu_oracle_images_per_s(args.steps, args.warmup, kind=args.net)
+    if outputs is not None:
+        outputs["sr"] = y
     out = {
         "impl": "reference", "metric": METRIC, "value": round(ips, 4), "unit": "images/s",
         "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": round(mean * 1e3, 2),
@@ -183,7 +206,7 @@ def barrier(world):
         torch.distributed.barrier()
 
 
-def run_infer(args):
+def run_infer(args, outputs=None):
     from vmambair_b200 import ops
     from vmambair_b200.engine import InferenceEngine
     rank, local, world = env_rank()
@@ -221,6 +244,8 @@ def run_infer(args):
             e.record(eng.stream)
     torch.cuda.synchronize(dev)
     barrier(world)
+    if outputs is not None:
+        outputs["sr"] = eng.y_dev.float().cpu()  # the last timed step's result, before the end-to-end runs below
     step_ms = [s.elapsed_time(e) for s, e in evs]
     total_ms = dist_max(sum(step_ms), world, dev)
     # ---- end-to-end through the public API: pinned host -> device -> net -> host, every step ----
@@ -300,13 +325,13 @@ def run_infer(args):
     return out
 
 
-def train_record(args):
-    """BASELINE configs[2] (the training step: the one path with a collective) as a sub-record of the default line, so the
-    driver's 1 -> 8 GPU sweep carries a training-scaling curve next to the collective-free inference one."""
+def train_record(args, outputs=None):
+    """BASELINE configs[2] (the training step: the one path with a collective) as a sub-record of the default line, so a
+    1 -> 8 GPU sweep carries a training-scaling curve next to the collective-free inference one."""
     from vmambair_b200.train_bench import run_train
     a = argparse.Namespace(**vars(args))
-    a.steps, a.warmup = min(args.steps, 10), 3
-    t = run_train(a, build_net, ClockSampler, env_rank, dist_max, barrier, peaks, sample_clocks=False)
+    a.warmup = 3
+    t = run_train(a, build_net, ClockSampler, env_rank, dist_max, barrier, peaks, sample_clocks=False, outputs=outputs)
     keep = ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "scaling", "dtype", "config", "e2e", "gpu_launches",
             "collective", "loss_last", "roofline")
     return {k: t[k] for k in keep}
@@ -327,9 +352,17 @@ def main():
     ap.add_argument("--config", type=int, default=2, choices=[2, 4, 5],
                     help="1-based index into BASELINE.json configs: 2 = VmambaIR-light SRx4 inference (default, the metric's config), "
                          "4 = deraining 4 x 3x256x256, 5 = RealSR 2 x 3x128x128 per GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path computed in its last timed step as DIR/<name>.npy, float32 (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    outputs = {} if args.dump_outputs else None
     if args.impl == "reference":
-        return run_reference(args)
+        run_reference(args, outputs)
+        if outputs:
+            dump_outputs(outputs, args.dump_outputs)
+        return
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device (the product has no CPU path); use --impl reference for the CPU oracle")
     rank, local, world = env_rank()
@@ -339,13 +372,15 @@ def main():
     try:
         if args.workload == "train":
             from vmambair_b200.train_bench import run_train
-            out = run_train(args, build_net, ClockSampler, env_rank, dist_max, barrier, peaks)
+            out = run_train(args, build_net, ClockSampler, env_rank, dist_max, barrier, peaks, outputs=outputs)
         else:
-            out = run_infer(args)
+            out = run_infer(args, outputs)
             if not args.no_train and args.config == 2:
-                out["train"] = train_record(args)
+                out["train"] = train_record(args, outputs)
         if rank == 0:
             print(json.dumps(out), flush=True)
+            if outputs is not None:
+                dump_outputs(outputs, args.dump_outputs)
     finally:
         if world > 1:
             torch.distributed.destroy_process_group()

@@ -1,7 +1,7 @@
 """Selective-scan backward at the north-star shape with and without the dB/dC reduction (VMB_BWD_NORED=1 skips the smem read-back +
 red.global of the group reduction): what that stage costs."""
 import json, os, sys
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from vmambair_b200 import ops
 from tools.scan_bench import bench

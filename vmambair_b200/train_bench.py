@@ -17,8 +17,9 @@ B_PER_GPU = 4
 H = W = 64
 
 
-def run_train(args, build_net, ClockSampler, env_rank, dist_max, barrier, peaks, sample_clocks=True):
-    """-> the JSON record (dict) of the training workload on this rank's GPU; the process group is the caller's."""
+def run_train(args, build_net, ClockSampler, env_rank, dist_max, barrier, peaks, sample_clocks=True, outputs=None):
+    """-> the JSON record (dict) of the training workload on this rank's GPU; the process group is the caller's.
+    outputs (a dict) receives the loss of the last timed step and the parameters after it."""
     from . import archs, ops
     from .optim import FlatAdam
     rank, local, world = env_rank()
@@ -114,10 +115,13 @@ def run_train(args, build_net, ClockSampler, env_rank, dist_max, barrier, peaks,
     s, e = torch.cuda.Event(True), torch.cuda.Event(True)
     s.record()
     for _ in range(K):
-        step(lq, gt)
+        loss = step(lq, gt)
     e.record()
     torch.cuda.synchronize(dev)
     barrier(world)
+    if outputs is not None:  # before the end-to-end steps below update the parameters again
+        outputs["train_loss"] = loss.detach().float().view(1).cpu()
+        outputs["train_params"] = opt.flat_param.cpu()
     total_ms = dist_max(s.elapsed_time(e), world, dev)
     # collective share: the all-reduce alone, timed on the device
     ar_ms = 0.0
